@@ -108,6 +108,26 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_ELEMS = 2 ** 22     # per array: the three dumped arrays stay under 64 MiB of float32 together
+
+
+def output_sample(t, seed):
+    """float32 host copy of `t`: the whole tensor when it has at most DUMP_ELEMS elements, else DUMP_ELEMS elements at
+    seeded flat indices, so that runs with the same arguments dump the same elements."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= DUMP_ELEMS:
+        return t.detach().float().cpu().numpy()
+    idx = torch.randint(flat.numel(), (DUMP_ELEMS,), generator=torch.Generator().manual_seed(seed))
+    return flat[idx.to(flat.device)].float().cpu().numpy()
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def randomize_zero_init_(model, std=0.02, seed=1234):
     """Quirk Q8: zero-init projections / identity gates would make most of the trunk an identity."""
     g = torch.Generator().manual_seed(seed)
@@ -234,11 +254,7 @@ def run_reference(args, rank, world):
         warm += 1
         if time.perf_counter() - t_start > budget * 0.3:
             break
-    times = []
-    for _ in range(args.steps):
-        times.append(step())
-        if time.perf_counter() - t_start > budget:
-            break
+    times = [step() for _ in range(args.steps)]
     t_blk = sum(times) / len(times)
     fwd = t_blk * CFG["depth"]
     val = N_RES * N_RES / fwd
@@ -349,7 +365,7 @@ def run_ours(args, rank, world, local_rank):
             flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            fn()
+            last = fn()
             b.record()
             b.synchronize()
             total += a.elapsed_time(b)
@@ -358,7 +374,7 @@ def run_ours(args, rank, world, local_rank):
             t = torch.tensor([total], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             total = t.item()
-        return total   # ms over `steps` steps, max over ranks
+        return total, last   # ms over `steps` steps, max over ranks; what the last step returned
 
     for _ in range(max(args.warmup, 3)):
         trunk_step()
@@ -368,13 +384,20 @@ def run_ours(args, rank, world, local_rank):
     clocks = ClockSampler(local_rank)
     clocks.start()
     l0 = lib.af2_launch_count()
-    ms_total = timed(trunk_step, args.steps)
+    ms_total, (x_out, m_out) = timed(trunk_step, args.steps)
     launches = int(lib.af2_launch_count() - l0)
     graphed = getattr(model.net, "_af2_graph", None) if world > 1 else None
     if graphed is not None and graphed.graph is not None:
         launches = graphed.launches_per_replay * args.steps      # the sharded forward is replayed as a CUDA graph
     clk = clocks.stop()
-    ms_e2e = timed(e2e_step, args.steps)
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        # copied before the e2e steps, which run the trunk again
+        dumps = {"pair": output_sample(x_out, 1), "msa": output_sample(m_out, 2)}
+    ms_e2e, _ = timed(e2e_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        dumps["distogram"] = output_sample(out_h, 3)
+        write_outputs(args.dump_outputs, dumps)
 
     # secondary, labelled number at N > 1 (SURVEY.md 8e fallback statement): N independent replicas, one unsharded sequence
     # per GPU, all ranks at the same time -- never the headline (`value` is the ONE sequence sharded over all ranks)
@@ -385,7 +408,7 @@ def run_ours(args, rank, world, local_rank):
         for _ in range(3):
             rep_step()
         rsteps = max(3, min(args.steps, 5))
-        ms_rep = timed(rep_step, rsteps) / rsteps
+        ms_rep = timed(rep_step, rsteps)[0] / rsteps
         replicas = {"value": world * N_RES * N_RES / (ms_rep * 1e-3), "unit": UNIT, "ms_per_step": ms_rep, "scaling": "weak",
                     "what": f"{world} independent sequences, one unsharded trunk forward per GPU, concurrently (secondary number)"}
 
@@ -509,7 +532,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="C2", choices=list(WORKLOADS),
                     help="BASELINE.json config shape (default C2 = the configuration the metric is quoted on)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): pair.npy and "
+                         "msa.npy from the trunk, distogram.npy from Alphafold2.forward; an array of more than "
+                         f"{DUMP_ELEMS} elements is replaced by that many of its elements at fixed seeded flat indices")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     set_workload(args.workload)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -8,8 +8,9 @@ It is a functional (no nn.Module) restatement in plain torch on the CPU, dtype-g
 
 Pinned: ``tests/test_oracle_golden.py`` checks every function here against fixtures in
 tests/golden/ that were produced by the unmodified reference (oracle/make_golden.py),
-and ``tests/test_oracle_vs_reference.py`` checks it live against the reference when
-/root/reference is present.  It must never be imported by ``alphafold2_b200``.
+and ``tests/test_oracle_vs_reference.py`` checks it against outputs the reference computed
+on seeded weights and inputs (oracle/make_golden_vs_reference.py).  It must never be
+imported by ``alphafold2_b200``.
 
 Two deliberate differences from the literal reference, both validated against it:
   * ``outer_mean(..., literal=False)`` contracts over the MSA axis with an einsum instead of
@@ -311,6 +312,18 @@ def randomize_zero_init_(state: W, std: float = 0.02, seed: int = 1234) -> W:
         elif bool((t == 1).all()) and (".gating." in k or "_gate." in k):
             t.copy_(1.0 + torch.randn(t.shape, generator=g) * std)
     return state
+
+
+def seeded_tensors(spec: Dict[str, tuple], seed: int) -> W:
+    """spec {name: (shape, mean, std)} -> {name: fp32 tensor of N(mean, std)}, drawn in spec order from one seeded
+    generator.  Lets a fixture pin weights and inputs by their statistics instead of storing them."""
+    g = torch.Generator().manual_seed(seed)
+    return {k: torch.randn(tuple(shape), generator=g) * std + mean for k, (shape, mean, std) in spec.items()}
+
+
+def sample_index(numel: int, k: int, seed: int) -> Tensor:
+    """A fixed, seeded choice of min(k, numel) flat indices, for fixtures that keep a sample of a larger output."""
+    return torch.randperm(numel, generator=torch.Generator().manual_seed(seed))[:k]
 
 
 def evoformer_flops_per_block(N: int, S: int, d: int, H: int, dh: int) -> float:
