@@ -57,6 +57,7 @@ _SIGNATURES = {
     "af2_abi_version": (ci, []),
     "af2_check_device": (ci, []),
     "af2_set_proj_mode": (None, [ci]),
+    "af2_set_ff_fused": (None, [ci]),
     "af2_debug_proj_trace": (ci, [C.POINTER(C.c_longlong)]),
     "af2_debug_attn_trace": (ci, [C.POINTER(C.c_longlong)]),
     "af2_launch_count": (C.c_ulonglong, []),

@@ -15,6 +15,7 @@
 #include "attention_tc.cuh"
 #include "chan2tok_tma.cuh"
 #include "gemm_tc.cuh"
+#include "ff_tc.cuh"
 #include "proj_tc.cuh"
 #include "simt_kernels.cuh"
 #include "strict_kernels.cuh"
@@ -604,6 +605,77 @@ int launch_attention(const __nv_bfloat16* qkv, int heads, int dh, int n, int nba
 
 #include "proj_launch.inl"
 
+// 1 (default): FeedForward blocks that ff_tc_kernel takes run as that one fused launch; 0: LN->W1->GEGLU (proj_tc) + residual
+// GEMM, two launches (af2_set_ff_fused, AF2_FF_FUSED)
+int g_ff_fused = 1;
+
+// shapes the fused transition kernel takes: d = 128 / 256 (pair-MMA N = d, K = d in pairs of 64-wide k-blocks), whole 64-unit
+// hidden chunks, the per-256-row-tile W1 packing of the fused projection path
+bool ff_fused_ok(const af2_ff_weights* w, int d, int hidden) {
+  return g_ff_fused && g_proj_ctas == 2 && w->w_cat && w->w_ext && w->bn == 256 && (d == 128 || d == 256) &&
+         hidden % FF_CHUNK == 0 && aligned16(w->w2) && aligned16(w->b2);
+}
+
+int launch_ff_fused(const af2_ff_weights* w, float* x, long long T, int d, int hidden, cudaStream_t s) {
+  if (T <= 0) return AF2_OK;
+  if (!aligned16(x)) return fail(AF2_ERR_BAD_ARG, "feed_forward: x not 16-byte aligned");
+  using L = FfSmem;
+  static bool configured_dev[MAX_DEVICES] = {false};
+  static int max_clusters_dev[MAX_DEVICES] = {0};
+  int& max_clusters = max_clusters_dev[cur_dev()];
+  if (!configured_dev[cur_dev()]) {
+    CUDA_OK(cudaFuncSetAttribute(ff_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL));
+    cudaLaunchConfig_t qc;
+    memset(&qc, 0, sizeof(qc));
+    qc.gridDim = dim3(sm_count(), 1, 1); qc.blockDim = dim3(FF_THREADS, 1, 1); qc.dynamicSmemBytes = L::TOTAL;
+    cudaLaunchAttribute qa[1];
+    qa[0].id = cudaLaunchAttributeClusterDimension; qa[0].val.clusterDim.x = 2; qa[0].val.clusterDim.y = 1; qa[0].val.clusterDim.z = 1;
+    qc.attrs = qa; qc.numAttrs = 1;
+    int nc = 0;
+    if (cudaOccupancyMaxActiveClusters(&nc, ff_tc_kernel, &qc) != cudaSuccess || nc <= 0) { cudaGetLastError(); nc = sm_count() / 2; }
+    max_clusters = nc < sm_count() / 2 ? nc : sm_count() / 2;
+    configured_dev[cur_dev()] = true;
+  }
+  const int n1p = (hidden + 127) / 128 * 256;          // packed W1 rows (w_cat)
+  CUtensorMap tw1, tb1, tw2, tx;
+  {
+    unsigned long long dw[2] = {(unsigned long long)d, (unsigned long long)n1p};
+    unsigned long long sw[1] = {(unsigned long long)d * 2};
+    unsigned bw[2] = {64, 64};
+    AF2_TRY(make_tmap(&tw1, w->w_cat, 2, dw, sw, bw, CU_TENSOR_MAP_SWIZZLE_128B));
+    unsigned long long dx[2] = {16ull, (unsigned long long)n1p};
+    unsigned long long sx[1] = {32ull};
+    unsigned bx[2] = {16, 64};
+    AF2_TRY(make_tmap(&tb1, w->w_ext, 2, dx, sx, bx, CU_TENSOR_MAP_SWIZZLE_32B));
+    unsigned long long d2[2] = {(unsigned long long)hidden, (unsigned long long)d};
+    unsigned long long s2[1] = {(unsigned long long)hidden * 2};
+    unsigned b2[2] = {64, (unsigned)(d / 2)};
+    AF2_TRY(make_tmap(&tw2, w->w2, 2, d2, s2, b2, CU_TENSOR_MAP_SWIZZLE_128B));
+    unsigned long long dxr[2] = {(unsigned long long)d, (unsigned long long)T};
+    unsigned long long sxr[1] = {(unsigned long long)d * 4};
+    unsigned bxr[2] = {32, 32};
+    AF2_TRY(make_tmap(&tx, x, 2, dxr, sxr, bxr, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_DATA_TYPE_FLOAT32));
+  }
+  FfParams p;
+  memset(&p, 0, sizeof(p));
+  p.x = x; p.b2 = w->b2; p.T = T; p.d = d; p.hidden = hidden; p.inv_d = 1.0f / (float)d; p.eps = 1e-5f;
+  p.m_units = (int)((T + 255) / 256);
+  const int clusters = p.m_units < max_clusters ? p.m_units : max_clusters;
+  // algorithmic FLOPs of both Linear layers; bytes: x read + written once, both weight matrices once
+  const double flops = 2.0 * T * (double)d * hidden * 3;
+  const double bytes = (double)T * d * 8 + (double)n1p * d * 2 + (double)d * hidden * 2;
+  ProfScope ps(s, KC_GEMM_LINEAR, flops, bytes);
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3(clusters * 2, 1, 1); cfg.blockDim = dim3(FF_THREADS, 1, 1); cfg.dynamicSmemBytes = L::TOTAL; cfg.stream = s;
+  cudaLaunchAttribute at[2];
+  at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = g_pdl ? 2 : 1;
+  CUDA_OK(cudaLaunchKernelEx(&cfg, ff_tc_kernel, tw1, tb1, tw2, tx, p));
+  return AF2_OK;
+}
+
 // OuterMean normaliser of pair rows [row0, row0 + rows) of one batch element (quirk Q3): bit-packed kernel when the packed
 // mask fits in shared memory, else the byte-loop kernel
 int launch_outer_scale(const uint8_t* mask, float* scale, uint32_t* words, int row0, int rows, int S, int N, float eps, cudaStream_t s);
@@ -693,9 +765,11 @@ int af2_debug_attn_trace(long long* out) {
 }
 
 void af2_set_proj_mode(int ctas) { g_proj_ctas = ctas < 0 ? 2 : (ctas > 2 ? 2 : ctas); }
+void af2_set_ff_fused(int on) { g_ff_fused = on != 0; }
 
 int af2_check_device(void) {
   if (const char* e = getenv("AF2_PROJ_CTAS")) af2_set_proj_mode(atoi(e));
+  if (const char* e = getenv("AF2_FF_FUSED")) af2_set_ff_fused(atoi(e));
   if (const char* e = getenv("AF2_C2T_TMA")) g_c2t_tma = atoi(e) != 0;
   if (const char* e = getenv("AF2_PROJ_PRODTILES")) g_proj_prod_tiles = atof(e);
   if (const char* e = getenv("AF2_PROJ_BALANCE")) g_proj_balance = atoi(e) != 0;
@@ -743,6 +817,7 @@ int af2_feed_forward(const af2_ff_weights* w, float* x, long long tokens, int d,
   if (!w || !x) return fail(AF2_ERR_BAD_ARG, "feed_forward: null argument");
   if (d % 8 || hidden % 8) return fail(AF2_ERR_BAD_ARG, "feed_forward: d=%d and hidden=%d must be multiples of 8", d, hidden);
   if (tokens > 0x7fffffffLL) return fail(AF2_ERR_BAD_ARG, "feed_forward: too many tokens");
+  if (ff_fused_ok(w, d, hidden)) return launch_ff_fused(w, x, tokens, d, hidden, s);   // LN -> W1 -> GEGLU -> W2 -> residual, h on chip
   Arena ar(workspace, workspace_bytes);
   __nv_bfloat16* xn = ar.take<__nv_bfloat16>(tokens * d);
   __nv_bfloat16* hbuf = ar.take<__nv_bfloat16>(tokens * hidden);

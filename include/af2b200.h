@@ -35,6 +35,10 @@ int af2_check_device(void);
 /* 2 (default): LN->projection clusters run on the fused CTA-pair kernel; 1: its single-CTA variant; 0: unfused
  * LayerNorm + GEMM launches (also selectable with the environment variable AF2_PROJ_CTAS, read by af2_check_device) */
 void af2_set_proj_mode(int ctas);
+/* 1 (default): af2_feed_forward runs the whole block (LayerNorm -> Linear -> GEGLU -> Linear -> residual) as one fused kernel
+ * when the shape allows it (d = 128 or 256, hidden a multiple of 64, the fused projection path in mode 2); 0: two launches
+ * (fused LayerNorm -> Linear -> GEGLU, then the residual GEMM).  Also selectable with the environment variable AF2_FF_FUSED. */
+void af2_set_ff_fused(int on);
 /* debug aid: with AF2_PROJ_TRACE=1 in the environment the fused projection kernel records clock64 stamps of one CTA
  * (MMA issue, epilogue and producer progress per tile); this copies the 2048 stamps of the last launch to `out` */
 int af2_debug_proj_trace(long long* out);

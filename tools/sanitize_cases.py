@@ -1,5 +1,6 @@
 """Small cases for tools/gpu_sanitize.sh: one C1-shape EvoformerBlock (every fused kernel: CTA-pair projection, tcgen05
-attention with resident bias, per-channel GEMMs, TMA channel->token) and one attention with n > 256 (streamed bias)."""
+attention with resident bias, per-channel GEMMs, TMA channel->token), one fused feed-forward at d = 256 and one attention
+with n > 256 (streamed bias)."""
 import os
 import sys
 
@@ -24,6 +25,16 @@ if case in ("all", "block"):
     torch.cuda.synchronize()
     assert torch.isfinite(xo).all() and torch.isfinite(mo).all()
     print("block ok")
+if case in ("all", "ff"):
+    # fused transition kernel (ff_tc_kernel) at d = 256 with a ragged row count: partial last unit, clusters with 1 and 2 units
+    ff = A.FeedForward(dim=256)
+    randomize_zero_init_(ff)
+    ff = ff.cuda().eval()
+    x = torch.randn(1, 3, 391, 256, device="cuda")
+    y = ff.add_to_(x.reshape(-1, 256).clone())
+    torch.cuda.synchronize()
+    assert torch.isfinite(y).all()
+    print("fused feed-forward ok")
 if case in ("all", "attn"):
     d, H, dh, n, rows = 128, 2, 64, 300, 3
     ax = A.AxialAttention(dim=d, heads=H, dim_head=dh, row_attn=True, col_attn=False, accept_edges=True)
